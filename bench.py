@@ -3,6 +3,7 @@
 roofline of the ray-march kernel and the CPU baseline beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3|cfg2|cfg2x2|cfg5_B] [--no-extras]
+    python bench.py ... --dump-outputs DIR    # also write the last timed tick's observation as DIR/<name>.npy
     python bench.py --impl reference ...      # the reference's own numba path (oracle/_ref), one process per host core
     torchrun ... bench.py --gpus N ...        # one rank per GPU; envs shard, no data-path collective
 
@@ -27,6 +28,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
 
 import numpy as np  # noqa: E402
 
@@ -61,6 +63,8 @@ EXTRA_WORKLOADS = ['cfg2', 'cfg2x2', 'cfg5_270', 'cfg5_540', 'cfg5_1080', 'cfg5_
 POSE_GAP = 23          # second agent 23 waypoints (~4.6 m) behind (SURVEY 8d)
 SEED = 12345
 FLUSH_BYTES = 256 << 20
+DUMP_SCAN_BYTES = 48 << 20      # --dump-outputs: scan rows beyond this are sampled (the whole dump stays under 64 MB)
+DUMP_SEED = 2024
 
 
 def config_dict(workload, world, sample=None):
@@ -302,8 +306,23 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------------------- GPU side
+def dump_outputs(sim, out_dir, torch):
+    """Writes the observation the last tick handed its caller (what f110_step_host copies out: scans, state, collisions,
+    done, lap times and counts) as out_dir/<name>.npy in float32 / float64, so that two builds can be compared output for
+    output.  When the scan block is larger than DUMP_SCAN_BYTES, a fixed seeded sample of agent rows stands for it."""
+    os.makedirs(out_dir, exist_ok=True)
+    NA, B = sim.scans.shape
+    n = min(NA, DUMP_SCAN_BYTES // (4 * B))
+    rows = np.arange(NA) if n == NA else np.sort(np.random.default_rng(DUMP_SEED).choice(NA, n, replace=False))
+    arrays = {'scans_sample': sim.scans[torch.from_numpy(rows).to(sim.device)],
+              'state': sim.state, 'collisions': sim.collisions, 'done': sim.done.to(torch.float32),
+              'lap_times': sim.lap_times, 'lap_counts': sim.lap_counts}
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v.cpu().numpy())
+
+
 def measure_workload(name, K, W, world, rank, dev, dmap, Ke, prof_ticks, f110, torch, dist, reduce_max_scalar,
-                     sampler_index=None, packed=False):
+                     sampler_index=None, packed=False, dump_dir=None):
     """One workload on this rank's GPU -> dict(value, ms_per_step, e2e, roofline, clocks, ...) (whole-job figures)."""
     w = WORKLOADS[name]
     N, A, B = w['num_envs'], w['num_agents'], w['num_beams']
@@ -357,6 +376,8 @@ def measure_workload(name, K, W, world, rank, dev, dmap, Ke, prof_ticks, f110, t
     clocks = sampler.stop() if sampler else None
     if world > 1:
         dist.barrier()
+    if dump_dir is not None:
+        dump_outputs(sim, dump_dir, torch)
     step_ms = np.array([a.elapsed_time(b) for a, b in zip(ev0, ev1)])
     dev_ms_total = reduce_max_scalar(float(step_ms.sum()), dev)
     value = K * NA * world / (dev_ms_total * 1e-3)
@@ -488,7 +509,8 @@ def run_b200(args):
     dmap = f110.DeviceMap.from_yaml(f110.maps.resolve_map_path('example_map'), '.png', dev)
     common = dict(world=world, rank=rank, dev=dev, dmap=dmap, f110=f110, torch=torch, dist=dist,
                   reduce_max_scalar=reduce_max_scalar)
-    main = measure_workload(args.workload, K, W, Ke=min(K, 200), prof_ticks=20, sampler_index=local_rank, packed=True, **common)
+    main = measure_workload(args.workload, K, W, Ke=min(K, 200), prof_ticks=20, sampler_index=local_rank, packed=True,
+                            dump_dir=args.dump_outputs if rank == 0 else None, **common)
 
     # optional NCCL observation all-gather for a single-process trainer (SURVEY 8e), timed OFF the step path
     gather = None
@@ -571,7 +593,11 @@ def main():
     ap.add_argument('--cpu-seconds', type=float, default=10.0)
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='skip the other BASELINE configs (1 GPU only)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the observation of the last one (rank 0) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == 'reference':

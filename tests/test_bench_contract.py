@@ -1,10 +1,13 @@
-"""bench.py contract (CPU): the reference arm runs here (the unmodified numba reference from oracle/_ref or
-/root/reference, one process per core; the oracle C port beside it) and prints one JSON line with the agreed keys whose
-`config` is key-identical to the CUDA arm's; the committed bench lines of the CUDA arm carry every key of the contract."""
+"""bench.py contract.  CPU: the reference arm (the unmodified numba reference when its modules are present, one process per
+core; the oracle C port beside it) prints one JSON line with the agreed keys whose `config` is key-identical to the CUDA
+arm's; the committed bench lines of the CUDA arm carry every key of the contract.  GPU: --dump-outputs is reproducible."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..')
 BASE_KEYS = ('metric', 'value', 'unit', 'n_gpus', 'steps', 'warmup', 'ms_per_step', 'higher_is_better', 'scaling',
@@ -75,3 +78,25 @@ def test_committed_round2_bench_line():
     assert c['kind'] == 'reference' and c['cores'] >= 1 and 0 < c['value'] < c['port_value']
     ref = json.load(open(os.path.join(ROOT, 'profiles', 'r2', 'bench_reference_arm_final.json')))
     assert ref['impl'] == 'reference' and ref['config'] == d['config'] and ref['cpu_baseline']['kind'] == 'reference'
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_exactly(tmp_path):
+    """--dump-outputs writes the last timed tick's observation (float32 / float64, under 64 MB with the flagship's scan
+    block sampled); the same arguments give the same arrays bit for bit, and one more timed step changes them."""
+    def run(steps, name):
+        out = tmp_path / name
+        r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', str(steps), '--warmup', '3', '--no-cpu',
+                            '--no-extras', '--dump-outputs', str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads([l for l in r.stdout.splitlines() if l.strip()][-1])
+        assert d['steps'] == steps and d['gpu_launches'] == 3 * steps
+        return {f[:-4]: np.load(out / f) for f in sorted(os.listdir(out))}
+    a, b, c = run(3, 'a'), run(3, 'b'), run(4, 'c')
+    assert set(a) == {'scans_sample', 'state', 'collisions', 'done', 'lap_times', 'lap_counts'}
+    assert sum(v.nbytes for v in a.values()) < 64e6
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert a['state'].shape == (7, 32768) and a['scans_sample'].shape[1] == 1080
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    assert not np.array_equal(a['state'], c['state'])
