@@ -10,6 +10,7 @@ from .env import F110Env                                              # noqa: F4
 from . import kernels, maps, trackgen                                 # noqa: F401
 from .kernels import ScanSimulator2D                                  # noqa: F401
 from .planner import PurePursuitPlanner                               # noqa: F401
+from .render import RenderView                                        # noqa: F401
 
-__all__ = ['F110Env', 'Simulator', 'Integrator', 'ScanSimulator2D', 'PurePursuitPlanner', 'DeviceMap', 'DeviceBeams', 'kernels', 'maps',
-           'trackgen']
+__all__ = ['F110Env', 'Simulator', 'Integrator', 'ScanSimulator2D', 'PurePursuitPlanner', 'DeviceMap', 'DeviceBeams', 'RenderView',
+           'kernels', 'maps', 'trackgen']

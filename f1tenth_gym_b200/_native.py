@@ -58,6 +58,14 @@ class F110HostObs(C.Structure):
                 ('lap_times', _dp), ('lap_counts', _dp), ('scans_u24', _dp)]
 
 
+class F110View(C.Structure):
+    _fields_ = [('width', C.c_int32), ('height', C.c_int32), ('channels', C.c_int32), ('camera', C.c_int32),
+                ('center_x', C.c_double), ('center_y', C.c_double), ('metres_per_pixel', C.c_double),
+                ('draw_scan', C.c_int32), ('palette', (C.c_uint8 * 3) * 8),
+                ('wx', _dp), ('wy', _dp), ('num_waypoints', C.c_int32),
+                ('table_start', _dp), ('num_tables', C.c_int32), ('env_table', _dp)]
+
+
 # name -> (restype, argtypes); this table is also what tests use to check that every symbol declared
 # in include/f110_b200.h is exported.
 _P = C.POINTER
@@ -93,6 +101,7 @@ SIGNATURES = {
     'f110_rasterize_track': (C.c_int, [_dp, C.c_int32, C.c_double, C.c_double, C.c_int32, C.c_int32, _dp, _dp, _dp]),
     'f110_scan_noise': (C.c_int, [_dp, C.c_int64, C.c_double, C.c_uint64, C.c_uint64, _dp]),
     'f110_pack_scans_u24': (C.c_int, [_dp, C.c_int64, _dp, _dp]),
+    'f110_render': (C.c_int, [_P(F110Sim), _P(F110Map), _P(F110Beams), _P(F110View), _dp, C.c_int32, _dp, _dp, _dp]),
 }
 
 # measurement / test aids exported by the library but not part of the public header

@@ -9,6 +9,8 @@
 //   k_tail         warp per agent       GJK vs. the other agents of the env, wall-hit state zeroing, opponent ray-cast inside the
 //                                       blocked-view window, collisions obs, then lap logic and auto-reset per env
 //                                       (k_finalize = the same without the env-level part, for f110_step)
+// Off the tick path, f110_render draws top-down frames of the state (render.cuh): k_render_frame (4 pixels per thread), then the
+// scan-endpoint and waypoint layers as stream-ordered scatter launches.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -fmad=false (no FMA contraction).
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -26,6 +28,7 @@
 #include "planner.cuh"
 #include "edt.cuh"
 #include "trackgen.cuh"
+#include "render.cuh"
 
 namespace f110 {
 
@@ -1854,6 +1857,68 @@ int f110_scan_noise(float *scans, int64_t count, double std_dev, uint64_t seed, 
     if (!scans || count <= 0) return F110_ERR_INVALID;
     k_scan_noise<<<(unsigned)((count + 255) / 256), 256, 0, (cudaStream_t)stream>>>(scans, count, std_dev, seed, offset);
     LAUNCH_CHECK("k_scan_noise");
+    return F110_OK;
+}
+
+int f110_render(const f110_sim *sim, const f110_map *map, const f110_beams *beams, const f110_view *view,
+                const int32_t *viewers, int32_t num_frames, uint8_t *out, double *camera_out, void *stream) {
+    if (!sim || !view || !out || ((uintptr_t)out & 3)) return F110_ERR_INVALID;
+    if (sim->num_envs <= 0 || sim->num_agents <= 0 || !sim->state || !(sim->sim_length > 0) || !(sim->sim_width > 0))
+        return F110_ERR_INVALID;
+    if ((long long)sim->num_envs * sim->num_agents > 0x7FFFFFFFLL) return F110_ERR_INVALID;
+    const f110_view &v = *view;
+    if (v.width <= 0 || v.height <= 0 || v.width % 4 != 0 || (v.channels != 1 && v.channels != 3) ||
+        (v.camera != 0 && v.camera != 1) || !(v.metres_per_pixel > 0) || !isfinite(v.metres_per_pixel) ||
+        !isfinite(v.center_x) || !isfinite(v.center_y))
+        return F110_ERR_INVALID;
+    const long long groups = (long long)(v.width / 4) * v.height;
+    if (groups > 0x7FFFFFFFLL) return F110_ERR_INVALID;
+    if (num_frames <= 0 || (!viewers && num_frames != sim->num_envs)) return F110_ERR_INVALID;
+    if (v.draw_scan && (check_beams(beams) || !sim->scans || !sim->scan_pose || !sim->agent_poses)) return F110_ERR_INVALID;
+    if (v.num_waypoints < 0 || (v.num_waypoints > 0 && (!v.wx || !v.wy))) return F110_ERR_INVALID;
+    if (v.table_start && (v.num_tables <= 0 || !v.env_table)) return F110_ERR_INVALID;
+    const size_t smem = (size_t)sim->num_agents * F110_RENDER_CAR * sizeof(double);
+    if (smem > 200 * 1024) return F110_ERR_INVALID;
+    int rc;
+    if ((rc = check_map(map))) return rc;
+
+    RenderArgs r;
+    memset(&r, 0, sizeof(r));
+    r.dt = map->dt;
+    r.orig_x = map->orig_x; r.orig_y = map->orig_y; r.orig_c = map->orig_c; r.orig_s = map->orig_s;
+    r.resolution = map->resolution; r.inv_resolution = 1.0 / map->resolution;
+    r.x_max = map->width * map->resolution;          // `width * resolution` (laser_models.py:79), as in make_view
+    r.y_max = map->height * map->resolution;
+    r.map_h = map->height; r.map_w = map->width;
+    r.layer_stride = (unsigned long long)map->height * (unsigned long long)map->width;
+    r.env_layer = (map->num_layers > 1) ? sim->env_layer : nullptr;
+    r.state = sim->state;
+    r.num_envs = sim->num_envs; r.num_agents = sim->num_agents; r.ego_idx = sim->ego_idx;
+    r.length = sim->sim_length; r.width = sim->sim_width;
+    r.W = v.width; r.H = v.height; r.channels = v.channels; r.camera = v.camera;
+    r.center_x = v.center_x; r.center_y = v.center_y; r.mpp = v.metres_per_pixel;
+    memcpy(r.palette, v.palette, sizeof(r.palette));
+    r.viewers = viewers; r.num_frames = num_frames; r.out = out;
+
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned fy = num_frames < 65535 ? (unsigned)num_frames : 65535u;
+    const dim3 grid((unsigned)((groups + F110_RENDER_THREADS - 1) / F110_RENDER_THREADS), fy);
+    // fast_path (power-of-two resolution, unrotated origin): x * (1/res) is the same number as x / res
+    auto kf = map->fast_path ? k_render_frame<true> : k_render_frame<false>;
+    if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kf<<<grid, F110_RENDER_THREADS, smem, st>>>(r, camera_out);
+    LAUNCH_CHECK("k_render_frame");
+    if (v.draw_scan) {
+        const int B = beams->num_beams;
+        k_render_scan<<<dim3((B + F110_RENDER_THREADS - 1) / F110_RENDER_THREADS, fy), F110_RENDER_THREADS, 0, st>>>(
+            r, sim->scans, sim->scan_pose, sim->agent_poses, beams->scan_angles, B, map->max_range);
+        LAUNCH_CHECK("k_render_scan");
+    }
+    if (v.num_waypoints > 0) {
+        k_render_waypoints<<<dim3((v.num_waypoints + F110_RENDER_THREADS - 1) / F110_RENDER_THREADS, fy), F110_RENDER_THREADS, 0,
+                             st>>>(r, v.wx, v.wy, v.num_waypoints, v.table_start, v.num_tables, v.env_table);
+        LAUNCH_CHECK("k_render_waypoints");
+    }
     return F110_OK;
 }
 

@@ -11,6 +11,7 @@ Extensions: num_envs (None = single env, reference-shaped numpy/list outputs; in
 tensors (N,A,...) that are views of device buffers valid until the next step), num_beams, fov, device,
 scan_noise_std (reference default 0.01; 0 disables the noise for bit-reproducible parity runs).
 The gym 0.19 API with the non-standard reset(poses) is kept on purpose (SURVEY.md 8b).
+render(mode='rgb_array') draws top-down frames on the device (render.py); there is no 'human' window.
 """
 import numpy as np
 import torch
@@ -20,7 +21,7 @@ from .simulator import Integrator, Simulator
 
 
 class F110Env(object):
-    metadata = {'render.modes': ['human', 'human_fast']}
+    metadata = {'render.modes': ['human', 'human_fast', 'rgb_array']}
     render_callbacks = []
 
     def __init__(self, **kwargs):
@@ -145,9 +146,23 @@ class F110Env(object):
         self.sim.update_params(params, agent_idx=index)
 
     def add_render_callback(self, callback_func):
-        """f110_env.py:377-385 (kept for API compatibility; rendering itself is out of scope)."""
+        """f110_env.py:377-385 (kept for API compatibility; the callbacks expect a pyglet EnvRenderer and are not called by
+        render('rgb_array'))."""
         F110Env.render_callbacks.append(callback_func)
 
-    def render(self, mode='human'):
-        assert mode in ['human', 'human_fast']
-        raise NotImplementedError('f1tenth_gym_b200 has no renderer (pyglet/OpenGL GUI is out of scope).')
+    def render(self, mode='human', view=None, env_ids=None):
+        """f110_env.py:387-418.  mode='rgb_array' draws top-down frames on the device (render.RenderView, default the
+        reference window: 1000x800, fixed camera at the origin), each env seen from its ego: single-env mode returns an
+        (H, W, 3) uint8 numpy array, batched mode a (len(env_ids), H, W, 3) uint8 CUDA tensor of the envs env_ids (default
+        (0,): a reference-size frame is 2.4 MB).  'human' / 'human_fast' windows are not available."""
+        assert mode in F110Env.metadata['render.modes']
+        if mode != 'rgb_array':
+            raise NotImplementedError('f1tenth_gym_b200 has no renderer (pyglet/OpenGL GUI is out of scope).')
+        from .render import RenderView
+        view = RenderView.reference() if view is None else view
+        if not self.batched:
+            return self.sim.render(view)[0].cpu().numpy()
+        ids = torch.as_tensor((0,) if env_ids is None else env_ids, dtype=torch.int64).reshape(-1)
+        if ids.numel() == 0 or int(ids.min()) < 0 or int(ids.max()) >= self.num_envs:
+            raise ValueError('env_ids must be env indices in [0, %d)' % self.num_envs)
+        return self.sim.render(view, viewers=ids * self.num_agents + self.ego_idx)

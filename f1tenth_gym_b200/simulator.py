@@ -237,6 +237,7 @@ class Simulator(object):
             nat.ptr(self.march_cost), nat.ptr(self.march_order), nat.ptr(self.march_count), self.march_ipa,
             nat.ptr(self.march_rec), float(noise_std), int(seed) & 0xFFFFFFFFFFFFFFFF)
         self._graph = None
+        self._render_all = None      # viewers='all' of render(): every flat agent index, made on first use
         self._zeros_NA = torch.zeros((N, A), dtype=torch.float64, device=dev)     # obs['linear_vels_y'] (always 0, :606)
 
     # ------------------------------------------------------------------ configuration
@@ -514,6 +515,18 @@ class Simulator(object):
         nat.check(nat.lib().f110_step_profile(C.byref(self.c), C.byref(self._map_struct), C.byref(self.beams.c),
                                               nat.ptr(a), ms, _stream_ptr(self.device)))
         return float(ms[0]), float(ms[1]), float(ms[2])
+
+    def render(self, view, viewers=None, out=None, camera_out=None):
+        """Top-down frames of the current state on the device (render.py, C ABI f110_render): returns `out`, a uint8 CUDA tensor
+        (F, H, W, channels), allocated only when out is None.  viewers: None = one frame per env from its ego_idx, 'all' = one
+        per flat agent index env*A + agent, or F flat agent indices (an out-of-range index gives an all-0 frame).
+        camera_out (F, 4) fp64, optional, receives each frame's (cx, cy, cr, sr).  No host synchronisation."""
+        from . import render
+        if isinstance(viewers, str) and viewers == 'all':
+            if self._render_all is None:
+                self._render_all = torch.arange(self.num_envs * self.num_agents, dtype=torch.int32, device=self.device)
+            viewers = self._render_all
+        return render.render(self, view, viewers, out, camera_out)
 
     def lookups(self):
         return int(self.lookup_counter.item()) if self.lookup_counter is not None else None

@@ -272,6 +272,42 @@ int f110_edt(const uint8_t *occupied, int32_t height, int32_t width, double reso
 int f110_rasterize_track(const double *segments, int32_t num_segments, double wall_inner, double wall_outer, int32_t height,
                           int32_t width, uint8_t *occupied, double *dist2_out, void *stream);
 
+/* ---- headless renderer ------------------------------------------------------------------------ */
+
+/* What a frame shows (reference rendering.py / F110Env.render, f110_env.py:387-418, drawn without a window).  Every pixel
+ * gets a label: 0 free or off the map, 1 wall (the map cell under the pixel centre has dt == 0, found with the literal
+ * xy_2_rc of laser_models.py:55-86; an env of a stacked map reads its own layer), 2 the viewer's car, 3 another car of the
+ * viewer's env, 4 an endpoint of the viewer's last scan (draw_scan; ranges < max_range), 5 a waypoint; later layers win in
+ * that order from 1 to 5, except that the viewer's car wins over other cars.  Row 0 is the top row; pixel (r, c) has its
+ * centre at u = (c + 0.5 - 0.5 width) mpp, v = (0.5 height - r - 0.5) mpp camera metres, i.e. at world
+ * x = cx + (u cr - v sr), y = cy + (u sr + v cr).  camera 0 is a fixed window, (cx, cy) = center, (cr, sr) = (1, 0);
+ * camera 1 follows the viewer heading up, (cx, cy) = its (x, y) and (cr, sr) = (sin yaw, -cos yaw), from `state`.  A car
+ * covers the pixels whose centre lies inside the rectangle of get_vertices (collision_models.py:237-260).  A point layer
+ * lands on pixel c = floor(u / mpp + 0.5 width), r = floor(0.5 height - v / mpp) with (u, v) its camera coordinates, and
+ * is dropped outside the frame.  Walls differ from the reference on purpose: it draws 1-pixel points at the corners of the
+ * image pixels that are 0; here a frame fills the cells the simulator collides with (image pixels <= 128). */
+typedef struct {
+    int32_t width, height, channels, camera;   /* width % 4 == 0; channels 1 (label per pixel) | 3 (palette[label] RGB);
+                                                  camera 0 (fixed window) | 1 (viewer, heading up) */
+    double center_x, center_y, metres_per_pixel;   /* center: camera 0 only */
+    int32_t draw_scan;                          /* != 0: label 4 layer (needs `beams`) */
+    uint8_t palette[8][3];                      /* RGB of each label when channels == 3 */
+    const double *wx, *wy; int32_t num_waypoints;          /* device [num_waypoints]; NULL / 0: no waypoint layer */
+    const int32_t *table_start; int32_t num_tables; const int32_t *env_table;   /* optional planner layout
+                                                  (f110_pure_pursuit_tables): env e draws rows [table_start[t], table_start[t+1])
+                                                  of table t = env_table[e]; env_table holds num_envs entries (device i32);
+                                                  NULL: every env draws every row */
+} f110_view;
+
+/* Render num_frames frames into out [num_frames][height][width][channels] u8 (device).  viewers [num_frames] (device i32)
+ * holds the flat agent index each frame is drawn for, or is NULL: then num_frames == num_envs and frame e is env e seen from
+ * its ego_idx.  An out-of-range viewer gives an all-0 frame (and camera (0, 0, 0, 0)).  camera_out (device [num_frames][4]
+ * f64, optional) receives each frame's (cx, cy, cr, sr).  beams is read only with draw_scan.  Reads the simulation state,
+ * writes nothing but out / camera_out; no host synchronisation and no allocation, so it can be captured in a CUDA graph
+ * after f110_tick.  F110_ERR_NO_MAP when `map` has no table bound. */
+int f110_render(const f110_sim *sim, const f110_map *map, const f110_beams *beams, const f110_view *view,
+                const int32_t *viewers, int32_t num_frames, uint8_t *out, double *camera_out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
